@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- rays/s of the render_rays hot path (BASELINE.json metric) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--precision MODE] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--precision MODE] [--impl reference] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[1] -- a 400x400 lego-shape frame, 160 000
 synthetic camera rays, N_samples=64 + N_importance=64, 8x256 MLP, fp32-parity arithmetic,
@@ -19,6 +19,7 @@ roofline: the fine-pass field kernel (2/3 of all FLOPs) timed alone with CUDA ev
 cpu_baseline: the CPU oracle port (the reference is Python/torch; it cannot travel to the GPU
          box) on the host cores, on a bounded sample of the same rays.
 --impl reference: only the CPU arm, same JSON schema, "impl": "reference".
+--dump-outputs DIR: what render_rays returned in the last timed step (rank 0) as DIR/<key>.npy; see dump_outputs.
 """
 from __future__ import annotations
 
@@ -33,6 +34,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: the bench leaves it as build() left it
 
 import torch  # noqa: E402
 
@@ -222,6 +224,24 @@ def workload_config(n_gpus, precision):
 
 
 # ----------------------------------------------------------------------------- GPU arm
+DUMP_SAMPLE_ROWS = 32768
+
+
+def dump_outputs(out_dir, res):
+    """Write a render_rays result as out_dir/<key>.npy (float32), so that two builds can be compared output for output.
+    rgb_* / depth_* are written whole; of the per-sample opacity_* arrays (123 MB for the 160 000-ray frame) the rows of
+    a fixed seeded sample of DUMP_SAMPLE_ROWS rays, in ray order, the same rows in every run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    n = res["rgb_fine"].shape[0]
+    rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE_ROWS].sort().values
+    for k, v in res.items():
+        v = v.detach()
+        if k.startswith("opacity_"):
+            v = v[rows.to(v.device)]
+        np.save(os.path.join(out_dir, f"{k}.npy"), v.float().cpu().numpy())
+
+
 # ----------------------------------------------------------------------------- other BASELINE configs (extras)
 def _fresh_models(dev, NeRF, default_init_params):
     models = []
@@ -450,7 +470,10 @@ def main():
     ap.add_argument("--precision", default=os.environ.get("SINNERF_B200_BENCH_PRECISION", "auto"))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the configs[2]/[3]/[4] and stock-PyTorch rows")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what render_rays returned in the last timed step to DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     capture_stdout()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -501,11 +524,13 @@ def main():
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
     rendering.DRAW_UNUSED_NOISE = True     # keep the reference's randn draws (rendering.py:224)
 
-    def step(r):
+    def step(r, keep=None):
         k = gather.begin() if p2p else 0
         with torch.no_grad():
             res = rendering.render_rays(models, emb, r, N_SAMPLES, False, 0, 0, N_IMPORTANCE, 32768, True,
                                         precision=precision, pixel_scatter=gather.scatter(k, rank * n) if p2p else None)
+        if keep is not None:
+            keep["res"] = res
         pix = pack_pixels(res)
         if p2p:
             gather.commit(k)
@@ -546,7 +571,11 @@ def main():
     sampler = ClockSampler(local_rank) if rank == 0 else None
     if sampler:
         sampler.start()
-    total_ms = timed(lambda: step(rays_dev), args.steps)
+    # with --dump-outputs each timed step keeps its result (dropping the previous one); written after the timed steps
+    last = {} if args.dump_outputs and rank == 0 else None
+    total_ms = timed(lambda: step(rays_dev, last), args.steps)
+    if last is not None:
+        dump_outputs(args.dump_outputs, last.pop("res"))
 
     def e2e_step():
         r = rays_pinned.to(dev, non_blocking=True)

@@ -1,12 +1,12 @@
 #!/usr/bin/env python
 """Generate the committed golden fixtures by running the REFERENCE itself.
 
-Run in the build container only (needs /root/reference; the GPU box has none):
+Needs a checkout of the original SinNeRF repository (models/, datasets/, ckpts/room.ckpt):
 
-    python tests/golden/make_golden.py
+    SINNERF_REF=/path/to/SinNeRF python tests/golden/make_golden.py
 
 Imports the reference's own ``models/rendering.py``, ``models/nerf.py``
-(unmodified, from /root/reference) on CPU/fp32 and records inputs + outputs of
+(unmodified) on CPU/fp32 and records inputs + outputs of
 every stage of the hot path.  Nothing here is used at run time by the product;
 tests compare (a) the oracle and (b) the CUDA path against these files.
 
@@ -15,6 +15,7 @@ Outputs (tests/golden/):
                      as plain arrays (realistic weight statistics; SURVEY.md 2 #15)
   stages.npz         Embedding / NeRF.forward / sample_pdf / activations goldens
   render_*.npz       whole render_rays cases (rays, config, RNG tensors, outputs)
+  reference_cases.npz  the randomised cases of tests/test_oracle_vs_reference_live.py
 """
 import os
 import sys
@@ -22,7 +23,9 @@ import sys
 import numpy as np
 import torch
 
-REF = "/root/reference"
+REF = os.environ.get("SINNERF_REF", "")
+if not os.path.isdir(os.path.join(REF, "models")):
+    sys.exit("set SINNERF_REF to a checkout of the original SinNeRF repository")
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, REF)
@@ -181,9 +184,78 @@ def c1_full():
                 n_importance=0, white_back=False)
 
 
+def reference_cases():
+    """What tests/test_oracle_vs_reference_live.py compares the oracle with, on its inputs: render_rays of its
+    randomised cases, the test_time keys, sample_pdf on random bins / weights, and reference autograd.  Gradient
+    tensors above GRAD_FULL_MAX entries are kept as norm + seeded sample + seeded projections (file size)."""
+    from tests.test_oracle_vs_reference_live import CASES, GRAD_FULL_MAX, grad_probe
+    out = {}
+    for i, (shape, n, S, Ni, use_disp, perturb, noise_std, white_back, seed) in enumerate(CASES):
+        rays = synthetic.random_rays(shape, n, seed=seed)
+        models = [model_from(default_init_params(10 + seed)), model_from(default_init_params(20 + seed))]
+        emb = [Embedding(3, 10), Embedding(3, 4)]
+        with torch.no_grad():
+            torch.manual_seed(100 + seed)
+            res = render_rays(models, emb, rays, S, use_disp, perturb, noise_std, Ni, 1024, white_back, test_time=False)
+        out[f"render{i}_cfg"] = np.array([n, S, Ni, use_disp, perturb, noise_std, white_back, seed], dtype=np.float64)
+        out[f"render{i}_rays"] = np_(rays)
+        for k, v in res.items():
+            out[f"render{i}_out_{k}"] = np_(v)
+
+    rays = synthetic.random_rays("lego", 12, seed=9)
+    models = [model_from(default_init_params(1)), model_from(default_init_params(2))]
+    with torch.no_grad():
+        res = render_rays(models, [Embedding(3, 10), Embedding(3, 4)], rays, 64, False, 0, 0, 64, 1024, True, test_time=True)
+    out["testtime_rays"] = np_(rays)
+    for k, v in res.items():
+        out[f"testtime_out_{k}"] = np_(v)
+
+    for seed in (0, 1, 2):
+        g = torch.Generator().manual_seed(seed)
+        n, m, ni = 19, 23 + seed, 31
+        bins = torch.sort(torch.rand(n, m + 1, generator=g) * 4 + 2, dim=-1).values
+        w = torch.rand(n, m, generator=g) ** 3
+        w[0] = 0.0                                    # all-zero weights row (the eps path)
+        out[f"pdf{seed}_bins"], out[f"pdf{seed}_w"] = np_(bins), np_(w)
+        out[f"pdf{seed}_out"] = np_(sample_pdf(bins, w, ni, det=True))
+
+    rays = synthetic.random_rays("llff", 14, seed=21)
+    models = [model_from(default_init_params(31)).train(), model_from(default_init_params(32)).train()]
+    torch.manual_seed(77)
+    res = render_rays(models, [Embedding(3, 10), Embedding(3, 4)], rays, 32, False, 1.0, 1.0, 24, 1024, False, test_time=False)
+    g = torch.Generator().manual_seed(5)
+    proj = {k: torch.randn(v.shape, generator=g) for k, v in res.items()}
+    sum((res[k] * proj[k]).sum() for k in res).backward()
+    out["grad_rays"] = np_(rays)
+    for k, v in proj.items():
+        out[f"grad_proj_{k}"] = np_(v)
+    none = []
+    for which, m in (("coarse", models[0]), ("fine", models[1])):
+        for name, prm in m.named_parameters():
+            key = f"{which}/{name}"
+            if prm.grad is None:
+                none.append(key)
+                continue
+            gr = prm.grad.double().flatten()
+            out[f"gnorm_{key}"] = np.array(float(gr.norm()))
+            if gr.numel() <= GRAD_FULL_MAX:
+                out[f"grad_{key}"] = np_(prm.grad)
+            else:
+                idx, p = grad_probe(gr.numel(), key)
+                out[f"gsample_{key}"] = np_(prm.grad.flatten()[idx])
+                out[f"gproj_{key}"] = np_(gr @ p)
+    out["grad_none"] = np.array(none, dtype=str)
+    path = os.path.join(HERE, "reference_cases.npz")
+    np.savez_compressed(path, **out)
+    print("wrote", path, len(out), "arrays")
+
+
 def main():
     if "--only-c1-full" in sys.argv:
         c1_full()
+        return
+    if "--reference-cases-only" in sys.argv:
+        reference_cases()
         return
     room = load_room()
     if "--rays-only" in sys.argv:
@@ -266,6 +338,7 @@ def main():
     grad_golden(room)
     rays_golden()
     c1_full()
+    reference_cases()
 
 
 if __name__ == "__main__":
