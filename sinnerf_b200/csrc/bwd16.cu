@@ -14,7 +14,6 @@
 //   layers    : dH_{l-1} = dgrad16(dH_l, W_l) * mask(h_l);  dW_l, db_l = wgrad16(dH_l, h_l)          l = 8 .. 1
 // HBM per point: ~2.5 KB per 256-wide layer (fp32 version: ~5 KB), 4.5 KB of saved activations (8.9 KB).
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 #include "act16.cuh"
 #include "common.cuh"
@@ -213,11 +212,9 @@ int field_backward16(const float* const* params, float* const* grads, int new_ac
   auto M = [&](int l) { return mask + (size_t)l * 8 * (size_t)ppad; };   // ReLU mask of h_{l+1}
   // The gradient chain carries its fp16 rounding residual (a second plane) from dS down to dH_4; below that the
   // chain is hi-only: a weight gradient then sees at most 4 chained 11-bit roundings (measured <= 4e-4 rel-L2, parity
-  // bar 1e-3) and the four lowest hops move 1 KB per point instead of 2.  SNB_BWD16_LO = 0: hi-only everywhere
-  // (first-layer gradients ~6e-4), 2: residual planes all the way down (~2.4e-4 flat).
-  static const int lo_mode = getenv("SNB_BWD16_LO") ? atoi(getenv("SNB_BWD16_LO")) : 1;
-  const bool use_lo = lo_mode != 0;
-  const int lo_floor = lo_mode == 2 ? 0 : 4;       // dH_l has a residual plane for l >= lo_floor
+  // bar 1e-3) and the four lowest hops move 1 KB per point instead of 2.  DESIGN.md section 4.3 lists the measured
+  // alternatives.
+  constexpr int lo_floor = 4;                      // dH_l has a residual plane for l >= lo_floor
   int rc;
   if (cudaMemsetAsync(state, 0, kBwdStateFloats * sizeof(float), st) != cudaSuccess)
     return fail(SNB_ERR_CUDA, "field_backward16: cudaMemsetAsync failed");
@@ -240,7 +237,7 @@ int field_backward16(const float* const* params, float* const* grads, int new_ac
   }
   {
     Head16Args a{reinterpret_cast<const float4*>(g_raw), reinterpret_cast<const float4*>(raw), act + A.g, params[kRgbW],
-                 new_activation, w + B.ds, use_lo ? w + B.ds_lo : nullptr, w + B.hg, grads[kRgbB], grads[kSigmaB], state, P, ppad};
+                 new_activation, w + B.ds, w + B.ds_lo, w + B.hg, grads[kRgbB], grads[kSigmaB], state, P, ppad};
     long long tiles = ppad / 32, blocks = (tiles + 7) / 8;
     if (blocks > sm_count() * 4) blocks = sm_count() * 4;
     head_bwd16_kernel<<<(unsigned)blocks, 256, 0, st>>>(a);
@@ -264,9 +261,9 @@ int field_backward16(const float* const* params, float* const* grads, int new_ac
   // into h8: through W', plus the sigma head's term; ReLU mask of h8
   unsigned char* cur = w + B.dya;
   unsigned char* nxt = w + B.dyb;
-  unsigned char* cur_lo = use_lo ? w + B.dya_lo : nullptr;
-  unsigned char* nxt_lo = use_lo ? w + B.dyb_lo : nullptr;
-  if ((rc = run_dgrad16(w + B.ds, use_lo ? w + B.ds_lo : nullptr, 128, fold + kFoldW, 256, 0, M(7), g_raw + 3, 4, params[kSigmaW], cur,
+  unsigned char* cur_lo = w + B.dya_lo;
+  unsigned char* nxt_lo = w + B.dyb_lo;
+  if ((rc = run_dgrad16(w + B.ds, w + B.ds_lo, 128, fold + kFoldW, 256, 0, M(7), g_raw + 3, 4, params[kSigmaW], cur,
                         cur_lo, state, ST_AMAX_DS, ST_SCALE_DS, ST_L1_FOLD, ST_AMAX_H0 + 7, ST_SCALE_H0 + 7, P, st)))
     return rc;
   for (int l = 7; l >= 1; --l) {
@@ -278,7 +275,7 @@ int field_backward16(const float* const* params, float* const* grads, int new_ac
     } else {
       if ((rc = run_wgrad16(cur, 256, H(l - 1), 256, 256, grads[2 * l], ldw, 0, grads[2 * l + 1], sc, nullptr, nullptr, nullptr, ppad, st))) return rc;
     }
-    const bool lo_in = use_lo && l >= lo_floor, lo_out = use_lo && l - 1 >= lo_floor;
+    const bool lo_in = l >= lo_floor, lo_out = l - 1 >= lo_floor;
     if ((rc = run_dgrad16(cur, lo_in ? cur_lo : nullptr, 256, params[2 * l], ldw, l == 4 ? kXyzCh : 0, M(l - 1), nullptr, 0, nullptr,
                           nxt, lo_out ? nxt_lo : nullptr, state, ST_AMAX_H0 + l, ST_SCALE_H0 + l, ST_L1_L0 + l, ST_AMAX_H0 + l - 1,
                           ST_SCALE_H0 + l - 1, P, st)))

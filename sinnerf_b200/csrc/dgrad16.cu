@@ -11,7 +11,8 @@
 //   * the gradient CHAIN (dgrad -> dgrad) is carried as fp16 hi + lo planes (22 bits), so rounding does not
 //     accumulate over the 8 layers; the wgrad of each layer reads only the hi plane -- its error is ONE fp16
 //     rounding of that layer's gradient, whatever the depth (measured: hi-only chains reached 1.1e-3 on the first
-//     layer's weights, hi + lo 2e-4; the parity bar is 1e-3).  kLo = false is the hi-only variant (SNB_BWD16_LO=0);
+//     layer's weights, hi + lo 2e-4; the parity bar is 1e-3).  field_backward16 carries hi + lo down to dH_4 and
+//     runs the lower hops hi-only (kLoIn / kLoOut = false);
 //   * W^T as fp16 hi + lo; products hi*hi + lo*hi + hi*lo (2 without the lo plane);
 //   * the epilogue multiplies by the power-of-two ratio s_out / s_in, adds the sigma head's rank-1 term,
 //     applies the ReLU mask (bit words the forward wrote, 32 B per point), rounds to fp16 and writes cells of
@@ -305,12 +306,9 @@ int run_dgrad16(const void* dY, const void* dY_lo, int N, const float* W, int ld
     if (li) return launch_dgrad16<256, true, false>(a, st);
     if (!lo) return launch_dgrad16<256, false, false>(a, st);
   }
-  if (N == 128) {
-    if (li && lo) return launch_dgrad16<128, true, true>(a, st);
-    if (!li && !lo) return launch_dgrad16<128, false, false>(a, st);
-  }
+  if (N == 128 && li && lo) return launch_dgrad16<128, true, true>(a, st);
   if (!li && lo) return fail(SNB_ERR_INVALID, "run_dgrad16: a residual plane cannot be produced from a hi-only input chain");
-  return fail(SNB_ERR_INVALID, "run_dgrad16: unsupported reduction length %d", N);
+  return fail(SNB_ERR_INVALID, "run_dgrad16: no kernel for reduction length %d with residual planes in / out = %d / %d", N, li, lo);
 }
 
 }  // namespace snb

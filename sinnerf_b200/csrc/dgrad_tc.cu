@@ -2,7 +2,7 @@
 //
 //   dX[p][k] = ( sum_n dY[p][n] W[n][col_off + k]  +  extra[p] evec[k] ) * [mask[p][k] > 0]        k < 256
 //
-// (reference: autograd through models/nerf.py:105-148; the SIMT version is dgrad_kernel in
+// (reference: autograd through models/nerf.py:105-148; the layer walk that calls it is in
 // field_bwd.cu.)  dY (P, N) with N = 256 or 128, mask = sign bits of the saved post-ReLU input of
 // the layer (32 B per point, emitted by the wgrad kernel that reads that input anyway), extra/evec =
 // the sigma head's rank-1 term at h8.  dY and dX are plain row-major fp32.

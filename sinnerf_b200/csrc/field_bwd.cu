@@ -1,240 +1,21 @@
-// field_bwd.cu -- backward of the field MLP (reference: autograd through models/nerf.py:105-148):
-// the driver that walks the layers, the head kernel, the folded bottleneck, and the fp32 FFMA
-// versions of the two GEMMs.  The GEMMs themselves run on tensor cores (wgrad_tc.cu, dgrad_tc.cu).
+// field_bwd.cu -- backward of the field MLP over fp32 saved activations (reference: autograd through
+// models/nerf.py:105-148): the driver that walks the layers, the head kernel and the folded bottleneck.
+// The two GEMMs of every layer run on tensor cores (wgrad_tc.cu, dgrad_tc.cu).
 //
 // Per render pass, given g_raw (P,4) = dL/d[r,g,b,sigma] from composite_bwd:
 //   heads     : rgb head + its activation, direction-layer activation, sigma head  (head_bwd_kernel)
 //   dir layer : W' = Wd[:, :256] Wf (fold_weights_kernel); dW', db' by one wgrad against h8; the chain
 //               rule back to Wd, Wf, bf, bd is three P-independent products (unfold_grads_kernel)
-//   per layer : dW_l += dY_l^T X_l, db_l += sum dY_l          (run_wgrad -> wgrad_tc_kernel | wgrad_kernel)
-//               dX_l  = dY_l W_l  (x ReLU mask of the saved input, + sigma term at h8)
-//                                                              (run_dgrad -> dgrad_tc_kernel | dgrad_kernel)
+//   per layer : dW_l += dY_l^T X_l, db_l += sum dY_l                               (wgrad_tc_kernel)
+//               dX_l  = dY_l W_l  (x ReLU mask of the saved input, + sigma term at h8)  (dgrad_tc_kernel)
 // walking dir layer -> layers 8..1.  Nothing flows into rays, z or across sample_pdf (the reference
 // detaches it, models/rendering.py:311-313).
 //
-// Activations are plain (P, C) row-major fp32 tensors.  The FFMA kernels (SNB_BWD_SIMT=1) stream rows
-// with 16-byte cp.async copies; wgrad_kernel accumulates a 128x128 block of dW per CTA in registers
-// over a slice of P and finishes with atomics (split-P), dgrad_kernel is the forward tiling with W
-// used untransposed.  Their roofline is the FP32 FFMA pipe; the tensor-core versions are HBM-bound.
-#include <stdlib.h>
-
+// Activations are plain (P, C) row-major fp32 tensors.  The wgrad of a layer also leaves the sign bits
+// [X > 0] of its input in ws_m; the dgrad of the same layer reads them as its ReLU mask.
 #include "common.cuh"
 
 namespace snb {
-
-constexpr int BT = 256;  // threads
-
-__device__ __forceinline__ void cp16(void* smem, const void* gmem) {
-  const uint32_t a = (uint32_t)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(a), "l"(gmem));
-}
-__device__ __forceinline__ void cp_commit() { asm volatile("cp.async.commit_group;\n" ::); }
-template <int N>
-__device__ __forceinline__ void cp_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N)); }
-
-// ------------------------------------------------------------------------------------------
-// wgrad:  dW[n0+n][col_off + k] += sum_p dY[p][n0+n] * X[p][k0+k],  db[n0+n] += sum_p dY[p][n0+n]
-// grid = (N/128, ceil(K/128), splits); each CTA walks rows [split*rows_per, +rows_per) in 32-row stages.
-// ------------------------------------------------------------------------------------------
-constexpr int WG_ROWS = 16;
-struct WgradArgs {
-  const float* dY; int ldy;        // (P, ldy)
-  const float* X; int ldx;         // (P, ldx)
-  int K;                           // valid columns of X
-  float* dW; int ldw; int col_off; // dW (N, ldw): block lands at columns [col_off, col_off + K)
-  float* db;                       // nullable; written by k-block 0 only
-  long long P;
-  long long rows_per_split;
-};
-
-__global__ void __launch_bounds__(BT) wgrad_kernel(WgradArgs a) {
-  __shared__ __align__(16) float sY[2][WG_ROWS][128];
-  __shared__ __align__(16) float sX[2][WG_ROWS][128];
-  const int tid = threadIdx.x, tn = tid >> 4, tk = tid & 15;   // 16 x 16 threads, 8x8 outputs each
-  const int n0 = blockIdx.x * 128, k0 = blockIdx.y * 128;
-  const long long r_begin = (long long)blockIdx.z * a.rows_per_split;
-  const long long r_end = r_begin + a.rows_per_split < a.P ? r_begin + a.rows_per_split : a.P;
-  float acc[8][8];
-  float accb[8];
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    accb[i] = 0.f;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
-  }
-  const int kcols = a.K - k0 < 128 ? a.K - k0 : 128;   // valid X columns in this block (multiple of 4 by padding)
-  auto load_stage = [&](int buf, long long r0) {
-    // 32 rows x 128 floats from each operand = 1024 float4 each; 4 per thread per operand
-#pragma unroll
-    for (int v = tid; v < WG_ROWS * 32; v += BT) {
-      const int r = v >> 5, c4 = (v & 31) * 4;
-      const long long row = r0 + r;
-      float* dy = &sY[buf][r][c4];
-      float* dx = &sX[buf][r][c4];
-      if (row < r_end) {
-        cp16(dy, a.dY + row * a.ldy + n0 + c4);
-        if (c4 < kcols) cp16(dx, a.X + row * a.ldx + k0 + c4);
-        else *reinterpret_cast<float4*>(dx) = make_float4(0.f, 0.f, 0.f, 0.f);
-      } else {
-        *reinterpret_cast<float4*>(dy) = make_float4(0.f, 0.f, 0.f, 0.f);
-        *reinterpret_cast<float4*>(dx) = make_float4(0.f, 0.f, 0.f, 0.f);
-      }
-    }
-  };
-  if (r_begin < r_end) {
-    load_stage(0, r_begin);
-    cp_commit();
-    int buf = 0;
-    for (long long r0 = r_begin; r0 < r_end; r0 += WG_ROWS, buf ^= 1) {
-      if (r0 + WG_ROWS < r_end) {
-        load_stage(buf ^ 1, r0 + WG_ROWS);
-        cp_commit();
-        cp_wait<1>();
-      } else {
-        cp_wait<0>();
-      }
-      __syncthreads();
-#pragma unroll 4
-      for (int r = 0; r < WG_ROWS; ++r) {
-        const float4 y0 = *reinterpret_cast<const float4*>(&sY[buf][r][tn * 8]);
-        const float4 y1 = *reinterpret_cast<const float4*>(&sY[buf][r][tn * 8 + 4]);
-        const float4 x0 = *reinterpret_cast<const float4*>(&sX[buf][r][tk * 8]);
-        const float4 x1 = *reinterpret_cast<const float4*>(&sX[buf][r][tk * 8 + 4]);
-        const float y[8] = {y0.x, y0.y, y0.z, y0.w, y1.x, y1.y, y1.z, y1.w};
-        const float x[8] = {x0.x, x0.y, x0.z, x0.w, x1.x, x1.y, x1.z, x1.w};
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          if (tk == 0) accb[i] += y[i];
-#pragma unroll
-          for (int j = 0; j < 8; ++j) acc[i][j] = fmaf(y[i], x[j], acc[i][j]);
-        }
-      }
-      __syncthreads();
-    }
-  }
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    const int n = n0 + tn * 8 + i;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      const int k = k0 + tk * 8 + j;
-      if (k < a.K) atomicAdd(a.dW + (size_t)n * a.ldw + a.col_off + k, acc[i][j]);
-    }
-    if (a.db != nullptr && blockIdx.y == 0 && tk == 0) atomicAdd(a.db + n, accb[i]);
-  }
-}
-
-// ------------------------------------------------------------------------------------------
-// dgrad:  dX[p][k] = ( sum_n dY[p][n] * W[n][col_off + k] + extra[p] * evec[k] ) * [mask[p][k] > 0]
-// 128-row tile per CTA, K = 256 outputs, N = 256 or 128 reduction.
-// ------------------------------------------------------------------------------------------
-struct DgradArgs {
-  const float* dY; int N;          // (P, N)
-  const float* W; int ldw; int col_off;   // nn.Linear weight (N, ldw)
-  const float* mask;               // (P,256) saved input activation (ReLU mask), nullable
-  const float* extra; int extra_stride;   // nullable: per-row scalar (g_sigma = g_raw[:,3])
-  const float* evec;               // (256) sigma head weight
-  float* dX;                       // (P,256)
-  long long P;
-};
-
-struct DgradSmem {
-  float y[128][260];        // dY tile, row-major, padded
-  float w[2][16][256];      // weight slices W[n..n+15][col_off..+255]
-};
-
-__global__ void __launch_bounds__(BT, 1) dgrad_kernel(DgradArgs a) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  DgradSmem& s = *reinterpret_cast<DgradSmem*>(smem_raw);
-  const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
-  const long long ntiles = (a.P + 127) / 128;
-  for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-    const long long p0 = tile * 128;
-    // stage the dY tile
-    const int nvec = a.N / 4;
-    for (int v = tid; v < 128 * nvec; v += BT) {
-      const int r = v / nvec, c4 = (v - r * nvec) * 4;
-      if (p0 + r < a.P) cp16(&s.y[r][c4], a.dY + (p0 + r) * a.N + c4);
-      else *reinterpret_cast<float4*>(&s.y[r][c4]) = make_float4(0.f, 0.f, 0.f, 0.f);
-    }
-    auto load_w = [&](int buf, int n_base) {
-      for (int v = tid; v < 16 * 64; v += BT) {
-        const int r = v >> 6, c4 = (v & 63) * 4;
-        // W rows are ldw floats apart and col_off may be odd (skip layer: 63): scalar-safe path
-        const float* src = a.W + (size_t)(n_base + r) * a.ldw + a.col_off + c4;
-        if ((reinterpret_cast<uintptr_t>(src) & 15) == 0) cp16(&s.w[buf][r][c4], src);
-        else {
-          s.w[buf][r][c4] = src[0]; s.w[buf][r][c4 + 1] = src[1];
-          s.w[buf][r][c4 + 2] = src[2]; s.w[buf][r][c4 + 3] = src[3];
-        }
-      }
-    };
-    load_w(0, 0);
-    cp_commit();
-    float acc[8][16];
-#pragma unroll
-    for (int i = 0; i < 8; ++i)
-#pragma unroll
-      for (int j = 0; j < 16; ++j) acc[i][j] = 0.f;
-    const int nslices = a.N / 16;
-    for (int sl = 0; sl < nslices; ++sl) {
-      if (sl + 1 < nslices) {
-        load_w((sl + 1) & 1, (sl + 1) * 16);
-        cp_commit();
-        cp_wait<1>();
-      } else {
-        cp_wait<0>();
-      }
-      __syncthreads();
-      const float(*wb)[256] = s.w[sl & 1];
-#pragma unroll
-      for (int n4 = 0; n4 < 16; n4 += 4) {
-        float4 yv[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) yv[i] = *reinterpret_cast<const float4*>(&s.y[ty * 8 + i][sl * 16 + n4]);
-#pragma unroll
-        for (int nn = 0; nn < 4; ++nn) {
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const float4 b = *reinterpret_cast<const float4*>(&wb[n4 + nn][j * 64 + tx * 4]);
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-              const float y = nn == 0 ? yv[i].x : (nn == 1 ? yv[i].y : (nn == 2 ? yv[i].z : yv[i].w));
-              acc[i][j * 4 + 0] = fmaf(y, b.x, acc[i][j * 4 + 0]);
-              acc[i][j * 4 + 1] = fmaf(y, b.y, acc[i][j * 4 + 1]);
-              acc[i][j * 4 + 2] = fmaf(y, b.z, acc[i][j * 4 + 2]);
-              acc[i][j * 4 + 3] = fmaf(y, b.w, acc[i][j * 4 + 3]);
-            }
-          }
-        }
-      }
-      __syncthreads();
-    }
-    // epilogue: + g_sigma * w_sigma, ReLU mask of the saved activation, store
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-      const long long row = p0 + ty * 8 + i;
-      if (row >= a.P) continue;
-      const float ex = a.extra != nullptr ? a.extra[row * a.extra_stride] : 0.f;
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const int c = j * 64 + tx * 4;
-        float4 v = make_float4(acc[i][j * 4], acc[i][j * 4 + 1], acc[i][j * 4 + 2], acc[i][j * 4 + 3]);
-        if (a.extra != nullptr) {
-          const float4 e = *reinterpret_cast<const float4*>(a.evec + c);
-          v.x = fmaf(ex, e.x, v.x); v.y = fmaf(ex, e.y, v.y); v.z = fmaf(ex, e.z, v.z); v.w = fmaf(ex, e.w, v.w);
-        }
-        if (a.mask != nullptr) {
-          const float4 m = *reinterpret_cast<const float4*>(a.mask + row * 256 + c);
-          v.x = m.x > 0.f ? v.x : 0.f; v.y = m.y > 0.f ? v.y : 0.f;
-          v.z = m.z > 0.f ? v.z : 0.f; v.w = m.w > 0.f ? v.w : 0.f;
-        }
-        *reinterpret_cast<float4*>(a.dX + row * 256 + c) = v;
-      }
-    }
-    __syncthreads();
-  }
-}
 
 // ------------------------------------------------------------------------------------------
 // heads: one warp walks points; lanes own 4 of the 128 direction-layer units and 8 of the 256
@@ -325,51 +106,14 @@ __global__ void __launch_bounds__(256) head_bwd_kernel(HeadArgs a) {
 // ------------------------------------------------------------------------------------------
 // host: the whole MLP backward of one render pass
 // ------------------------------------------------------------------------------------------
-static int dev_sms() { return sm_count(); }
-
-// wgrad_tc.cu: the same contraction on tensor cores (bf16 hi/lo split, fp32 accumulate in TMEM)
+// wgrad_tc.cu: dW[:, col_off + k] += dY^T X, db += sum dY on tensor cores (bf16 hi/lo split, fp32 accumulate in
+// TMEM); x_pos_bits (nullable) receives [X > 0] for the dgrad of the same layer
 int run_wgrad_tc(const float* dY, int N, const float* X, int ldx, int K, float* dW, int ldw, int col_off, float* db,
                  uint32_t* x_pos_bits, long long P, cudaStream_t st);
-
-// SNB_BWD_SIMT=1 keeps the FFMA kernels (debugging / A-B timing); the tensor-core kernels are the default
-static bool bwd_simt() {
-  static const bool simt = getenv("SNB_BWD_SIMT") && atoi(getenv("SNB_BWD_SIMT")) != 0;
-  return simt;
-}
-
-// x_bits (nullable): where the tensor-core kernel leaves [X > 0] for the dgrad of the same layer
-static int run_wgrad(const float* dY, int N, const float* X, int ldx, int K, float* dW, int ldw, int col_off,
-                     float* db, uint32_t* x_bits, long long P, cudaStream_t st) {
-  if (!bwd_simt()) return run_wgrad_tc(dY, N, X, ldx, K, dW, ldw, col_off, db, x_bits, P, st);
-  WgradArgs a{dY, N, X, ldx, K, dW, ldw, col_off, db, P, 0};
-  const int nb = N / 128, kb = (K + 127) / 128;
-  int splits = (2 * dev_sms()) / (nb * kb);
-  if (splits < 1) splits = 1;
-  long long rows = (P + splits - 1) / splits;
-  rows = (rows + WG_ROWS - 1) / WG_ROWS * WG_ROWS;
-  splits = (int)((P + rows - 1) / rows);
-  a.rows_per_split = rows;
-  wgrad_kernel<<<dim3(nb, kb, splits), BT, 0, st>>>(a);
-  return check_launch("wgrad_kernel");
-}
-
-// dgrad_tc.cu: the same product on tensor cores (CTA pairs, W^T resident in shared memory)
+// dgrad_tc.cu: dX = (dY W[:, col_off:] + extra evec) x [mask_bits] on tensor cores (CTA pairs, W^T resident in
+// shared memory)
 int run_dgrad_tc(const float* dY, int N, const float* W, int ldw, int col_off, const uint32_t* mask_bits,
                  const float* extra, int extra_stride, const float* evec, float* dX, long long P, cudaStream_t st);
-
-// mask: the saved fp32 input of the layer (FFMA kernel); mask_bits: its sign bits (tensor-core kernel)
-static int run_dgrad(const float* dY, int N, const float* W, int ldw, int col_off, const float* mask,
-                     const uint32_t* mask_bits, const float* extra, int extra_stride, const float* evec, float* dX,
-                     long long P, cudaStream_t st) {
-  if (!bwd_simt()) return run_dgrad_tc(dY, N, W, ldw, col_off, mask_bits, extra, extra_stride, evec, dX, P, st);
-  static SmemOptIn optin;
-  if (int rc = ensure_smem(dgrad_kernel, optin, (int)sizeof(DgradSmem), "dgrad")) return rc;
-  DgradArgs a{dY, N, W, ldw, col_off, mask, extra, extra_stride, evec, dX, P};
-  const long long ntiles = (P + 127) / 128;
-  const int grid = (int)(ntiles < dev_sms() ? ntiles : dev_sms());
-  dgrad_kernel<<<grid, BT, sizeof(DgradSmem), st>>>(a);
-  return check_launch("dgrad_kernel");
-}
 
 // params / grads: 24 device pointers in state-dict order (SNB_N_PARAM_TENSORS); grads are accumulated into.
 // ------------------------------------------------------------------------------------------
@@ -446,37 +190,34 @@ int field_backward_fp32(const float* const* params, float* const* grads, int new
   {
     HeadArgs a{g_raw, raw, save_g, H(7), params[kRgbW], new_activation, ws_s,
                grads[kRgbW], grads[kRgbB], grads[kSigmaW], grads[kSigmaB], P};
-    const int grid = dev_sms() * 4;
+    const int grid = sm_count() * 4;
     head_bwd_kernel<<<grid, 256, 0, st>>>(a);
     if ((rc = check_launch("head_bwd_kernel"))) return rc;
   }
   // direction layer with the bottleneck folded in: X = [h8 (through W') | dir]
-  fold_weights_kernel<<<128, 256, 0, st>>>(params[18], params[16], ws_w);
-  if ((rc = check_launch("fold_weights_kernel"))) return rc;
-  if ((rc = run_wgrad(ws_s, 128, H(7), 256, 256, ws_w + kFoldDW, 256, 0, ws_w + kFoldDB, ws_m, P, st))) return rc;
-  if ((rc = run_wgrad(ws_s, 128, save_dir, kDirPad, kDirCh, grads[18], 283, 256, nullptr, nullptr, P, st))) return rc;
-  unfold_grads_kernel<<<392, 256, 0, st>>>(params[18], params[16], params[17], ws_w, grads[18], grads[19], grads[16],
-                                           grads[17]);
-  if ((rc = check_launch("unfold_grads_kernel"))) return rc;
+  if ((rc = launch_fold_weights(params[18], params[16], ws_w, st))) return rc;
+  if ((rc = run_wgrad_tc(ws_s, 128, H(7), 256, 256, ws_w + kFoldDW, 256, 0, ws_w + kFoldDB, ws_m, P, st))) return rc;
+  if ((rc = run_wgrad_tc(ws_s, 128, save_dir, kDirPad, kDirCh, grads[18], 283, 256, nullptr, nullptr, P, st))) return rc;
+  if ((rc = launch_unfold_grads(params[18], params[16], params[17], ws_w, grads[18], grads[19], grads[16], grads[17], st))) return rc;
   // into h8: through W', plus the sigma head's term; ReLU mask of h8
-  if ((rc = run_dgrad(ws_s, 128, ws_w + kFoldW, 256, 0, H(7), ws_m, g_raw + 3, 4, params[kSigmaW], ws_b, P, st))) return rc;
+  if ((rc = run_dgrad_tc(ws_s, 128, ws_w + kFoldW, 256, 0, ws_m, g_raw + 3, 4, params[kSigmaW], ws_b, P, st))) return rc;
   // trunk layers 8..2 (index l = 7..1): dY lives in cur, dX goes to nxt
   float* cur = ws_b;
   float* nxt = ws_a;
   for (int l = 7; l >= 1; --l) {
     const int ldw = l == 4 ? 319 : 256;
     if (l == 4) {
-      if ((rc = run_wgrad(cur, 256, save_enc, kXyzPad, kXyzCh, grads[2 * l], ldw, 0, grads[2 * l + 1], nullptr, P, st))) return rc;
-      if ((rc = run_wgrad(cur, 256, H(l - 1), 256, 256, grads[2 * l], ldw, kXyzCh, nullptr, ws_m, P, st))) return rc;
-      if ((rc = run_dgrad(cur, 256, params[2 * l], ldw, kXyzCh, H(l - 1), ws_m, nullptr, 0, nullptr, nxt, P, st))) return rc;
+      if ((rc = run_wgrad_tc(cur, 256, save_enc, kXyzPad, kXyzCh, grads[2 * l], ldw, 0, grads[2 * l + 1], nullptr, P, st))) return rc;
+      if ((rc = run_wgrad_tc(cur, 256, H(l - 1), 256, 256, grads[2 * l], ldw, kXyzCh, nullptr, ws_m, P, st))) return rc;
+      if ((rc = run_dgrad_tc(cur, 256, params[2 * l], ldw, kXyzCh, ws_m, nullptr, 0, nullptr, nxt, P, st))) return rc;
     } else {
-      if ((rc = run_wgrad(cur, 256, H(l - 1), 256, 256, grads[2 * l], ldw, 0, grads[2 * l + 1], ws_m, P, st))) return rc;
-      if ((rc = run_dgrad(cur, 256, params[2 * l], ldw, 0, H(l - 1), ws_m, nullptr, 0, nullptr, nxt, P, st))) return rc;
+      if ((rc = run_wgrad_tc(cur, 256, H(l - 1), 256, 256, grads[2 * l], ldw, 0, grads[2 * l + 1], ws_m, P, st))) return rc;
+      if ((rc = run_dgrad_tc(cur, 256, params[2 * l], ldw, 0, ws_m, nullptr, 0, nullptr, nxt, P, st))) return rc;
     }
     float* t = cur; cur = nxt; nxt = t;
   }
   // layer 1: weights only
-  return run_wgrad(cur, 256, save_enc, kXyzPad, kXyzCh, grads[0], 63, 0, grads[1], nullptr, P, st);
+  return run_wgrad_tc(cur, 256, save_enc, kXyzPad, kXyzCh, grads[0], 63, 0, grads[1], nullptr, P, st);
 }
 
 }  // namespace snb

@@ -500,7 +500,7 @@ struct TcParams {
   unsigned char* a_g;      // (Ppad,128)
   uint32_t* a_mask;        // (8, 8, Ppad)
   long long ppad;
-  int debug;   // timing experiments only (SNB_TC_DEBUG): 2 = epilogue skips math, 4 = no MMAs
+  int debug;   // SNB_TC_DEBUG; only bit 8 is read: record the clock64 trace below
 };
 
 // ---- debug trace (SNB_TC_DEBUG & 8): clock64 stamps of one slot of cluster 0's leader CTA
@@ -679,7 +679,6 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
       constexpr uint32_t kStepB = (2 * G::kRowsB * 16) >> 4;     // one K16 step inside a chunk, in 16-B units
       constexpr uint32_t kStepA = (2 * kTile * 16) >> 4;
       auto commit = [&](uint64_t* bar) { if (kCg == 2) mma2_commit(bar); else mma_commit(bar); };
-      const bool do_mma = !(p.debug & 4);
       uint32_t st = 0, ph_full = 0;            // ring position: stage and the parity of its `full` barrier
       for (long long slot = 0; slot < n_slots; ++slot) {
         const uint32_t slot_par = (uint32_t)slot & 1;    // enc_ready / dir_ready / d_drained complete once per slot
@@ -751,12 +750,12 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
           using I0 = std::integral_constant<int, 0>;
           using IM = std::integral_constant<int, c.mid>;
           using IS = std::integral_constant<int, c.steps>;
-          if (do_mma) issue_range(I0{}, IM{});
+          issue_range(I0{}, IM{});
           trace(tr, 512 + CI * 4 + 0);
           if (c.mid < c.steps) {            // the chunk spans two K quarters: the second arrives later
             wait_code(std::integral_constant<int, c.wait_mid>{}, std::integral_constant<int, 2>{});
             tc_fence_after();
-            if (do_mma) issue_range(IM{}, IS{});
+            issue_range(IM{}, IS{});
             trace(tr, 512 + CI * 4 + 1);
           }
           commit(&s.empty[st]);        // ring slot free (in both CTAs of a pair) once these MMAs retire
@@ -997,10 +996,6 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
           trace(tr, tb + 1);
           const int q = ch >> 1;                       // the 64-column quarter this thread's group belongs to
           const int c0 = h * kNh + ch * 32;            // output columns == next layer's k
-          if (p.debug & 2) {
-            if (h == 0) { mbar_wait(&s.a_free, ph_free); ph_free ^= 1; }
-            tc_fence_before(); signal(&s.a_ready[h * 2 + q]); continue;
-          }
           uint32_t v[32];
           tmem_ld32(tbase + lane_base + kColD + c0, v);
           tmem_wait_ld();

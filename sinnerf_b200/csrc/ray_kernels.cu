@@ -1036,8 +1036,7 @@ int launch_composite(const float* raw, int raw_channels, const float* z, const f
                                         ? SNB_OK : fail(SNB_ERR_CUDA, "cudaMemsetAsync(loss)");
     return SNB_OK;
   }
-  static const bool warp_per_ray = getenv("SNB_COMPOSITE_WARP_PER_RAY") != nullptr;   // A/B timing of the two mappings
-  if (composite_quad_ok(S, raw, z, noise, w) && !warp_per_ray) {
+  if (composite_quad_ok(S, raw, z, noise, w)) {
     // four samples per thread: the ray's S/4 threads in a lane group of L = 8 / 16 / 32, 32 / L rays per warp pass
     const int L = S <= 32 ? 8 : (S <= 64 ? 16 : 32);
     int grid = grid_for(n_rays, 8 * (32 / L), device_sms() * 8);
@@ -1060,8 +1059,7 @@ int launch_composite_bwd(const float* raw, const float* z, const float* rays, co
                           int S, float* g_raw, const SnbLossSpec* loss, const float* out_rgb, const float* out_depth,
                           const float* g_loss, float* g_amax, cudaStream_t st) {
   if (n_rays == 0) return SNB_OK;
-  static const bool warp_per_ray = getenv("SNB_COMPOSITE_WARP_PER_RAY") != nullptr;
-  if (composite_quad_ok(S, raw, z, noise, g_w) && (reinterpret_cast<uintptr_t>(g_raw) & 15) == 0 && !warp_per_ray) {
+  if (composite_quad_ok(S, raw, z, noise, g_w) && (reinterpret_cast<uintptr_t>(g_raw) & 15) == 0) {
     const int L = S <= 32 ? 8 : (S <= 64 ? 16 : 32);
     const int grid = grid_for(n_rays, 8 * (32 / L), device_sms() * 6);
     const LossSpec ls = make_loss_spec(loss);

@@ -2,8 +2,8 @@
 //
 //   dW[n][col_off + k] += sum_p dY[p][n] * X[p][k]      db[n] += sum_p dY[p][n]
 //
-// (reference: autograd of `nn.Linear` inside models/nerf.py:105-148; the SIMT version of the same
-// contraction is wgrad_kernel in field_bwd.cu.)  dY (P, N) and X (P, ldx) are the plain row-major
+// (reference: autograd of `nn.Linear` inside models/nerf.py:105-148; the layer walk that calls it
+// is in field_bwd.cu.)  dY (P, N) and X (P, ldx) are the plain row-major
 // fp32 tensors the training forward / the dgrad chain leave in HBM.
 //
 // As an MMA the reduction runs over POINTS:  D[m = out feature][n' = in feature] += A[m][p] B[n'][p],

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """rel-L2 of every parameter gradient (CUDA path vs autograd through the CPU oracle with the CUDA path's
-fine depths injected).  SNB_BWD_SIMT=1 selects the FFMA backward, SINNERF_B200_PRECISION the forward.
+fine depths injected).  SINNERF_B200_PRECISION selects the forward.
 
     python tools/grad_error.py [n_rays] [weights: seed|room] [loss: sum|proj]
 """
@@ -49,7 +49,7 @@ of = {k: v.clone().requires_grad_(True) for k, v in pf.items()}
 ref = orc.render_rays(oc, of, rays, N_samples=64, N_importance=64, noise_std=0.0, white_back=True,
                       z_fine_override=out["_inter"]["z_fine"].detach().cpu())
 loss_of(ref, proj).backward()
-print(f"n_rays={n} weights={weights} loss={loss_kind} SNB_BWD_SIMT={os.environ.get('SNB_BWD_SIMT', '0')} "
+print(f"n_rays={n} weights={weights} loss={loss_kind} "
       f"precision={os.environ.get('SINNERF_B200_PRECISION', 'default')}")
 for name, ref_p, model in (("coarse", oc, models[0]), ("fine", of, models[1])):
     got = dict(model.named_parameters())

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Per-tensor rel-L2 of the parameter gradients of the fp16-storage training path against the fp32-storage path
-(round-1 kernels) on the same rays / projections.  SNB_BWD16_LO=0 selects the hi-only gradient chain.
+(round-1 kernels) on the same rays / projections.
 
     python tools/grad_error16.py [n_rays] [seed|room]
 """
@@ -47,7 +47,7 @@ for storage in ("fp32", "fp16"):
         proj = {k: torch.randn(v.shape, generator=gp).to(dev) for k, v in out.items()}
     sum((out[k] * proj[k]).sum() for k in proj).backward()
     grads[storage] = [{k: p.grad.detach().double().cpu() for k, p in m.named_parameters()} for m in models]
-print(f"{which} weights, {n} rays, SNB_BWD16_LO={os.environ.get('SNB_BWD16_LO', '1')}: rel-L2 of fp16-storage gradients vs fp32-storage")
+print(f"{which} weights, {n} rays: rel-L2 of fp16-storage gradients vs fp32-storage")
 for name, a, b in (("coarse", grads["fp16"][0], grads["fp32"][0]), ("fine", grads["fp16"][1], grads["fp32"][1])):
     for k in a:
         nb = float(b[k].norm())

@@ -5,7 +5,7 @@ import os
 import subprocess
 import sys
 
-os.environ["SNB_TC_DEBUG"] = str(8 | int(os.environ.get("SNB_TC_DEBUG_EXTRA", "0")))
+os.environ["SNB_TC_DEBUG"] = "8"
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.argv = [sys.argv[0], "--precision", sys.argv[1] if len(sys.argv) > 1 else "f16x3", "--rays", "8000", "--iters", "1"]
 exec(open(os.path.join(os.path.dirname(__file__), "time_field.py")).read())
