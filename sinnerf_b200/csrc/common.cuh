@@ -68,7 +68,7 @@ struct PackedHeader {
   uint32_t magic;      // 'SNBW'
   int32_t precision;   // SNB_PREC_*
   int32_t new_activation;
-  int32_t cta_group;
+  int32_t reserved0;   // unused; keeps the fields below at their offsets (tests read `dirty` as word 4)
   // snb_refresh_weights: a position-dependent 64-bit checksum of the 24 fp32 parameter tensors the image was
   // packed from.  The check kernel recomputes it on the device and sets `dirty`; the pack kernels of a
   // refresh return immediately when it is 0 -- no host round trip, and in-place updates that bypass

@@ -62,7 +62,7 @@ namespace snb {
 using namespace umma;
 
 // ------------------------------------------------------------------ geometry
-constexpr int kTile = 128;             // points per CTA tile (MMA M = 128 * cta_group)
+constexpr int kTile = 128;             // points per CTA tile (an MMA spans both tiles of the pair: M = 256)
 constexpr int kNh = 128;               // output columns per MMA (N); a 256-wide layer is two halves
 constexpr int kEpiWarps = 16;          // warps 0..15: prologue / epilogue (4 per TMEM lane quadrant)
 constexpr int kMmaWarp = 16, kLoadWarp = 17;
@@ -70,16 +70,13 @@ constexpr int kEncWarp0 = 18, kEncWarps = 2;   // positional encodings of the NE
 constexpr int kThreads = (kEncWarp0 + kEncWarps) * 32;   // 640: <= 102 registers per thread (96 used)
 constexpr uint32_t kColD = 0, kColAhi = 256, kColAlo = 384;
 
-// per cta_group geometry: a chunk is 128 output rows x (16 * steps) of K, steps <= kMaxSteps; each
-// CTA of the group holds kRowsB = 128 / cg of those rows
-template <int kCg>
-struct Geo {
-  static constexpr int kKc = kCg == 2 ? 128 : 32;            // K per full chunk
-  static constexpr int kRowsB = kNh / kCg;
-  static constexpr int kMaxSteps = kKc / 16;
-  static constexpr uint32_t kStepBytes = kRowsB * 16 * 2;    // one K16 step of one of {hi, lo} of a CTA's share
-  static constexpr uint32_t kPartBytesMax = kStepBytes * kMaxSteps;
-};
+// weight chunks: a chunk is 128 output rows x (16 * steps) of K, steps <= kMaxSteps; each CTA of the
+// pair holds kRowsB = 64 of those rows
+constexpr int kKc = 128;                                    // K per full chunk
+constexpr int kRowsB = kNh / 2;
+constexpr int kMaxSteps = kKc / 16;
+constexpr uint32_t kStepBytes = kRowsB * 16 * 2;            // one K16 step of one of {hi, lo} of a CTA's share
+constexpr uint32_t kPartBytesMax = kStepBytes * kMaxSteps;
 
 enum { SRC_ENC = 0, SRC_HID = 1, SRC_DIR = 2 };
 // WAIT_A0..A3: the previous layer's epilogue has stored output columns [64q, 64q+64) (= this layer's K
@@ -116,7 +113,6 @@ struct ChunkTable {
 
 // order inside a layer: half a (enc, hid k 0..255) -> D_a | half b (enc, hid k 0..127) -> A[k0] free |
 // (hid k 128..255) -> D_b
-template <int KC>
 __host__ __device__ constexpr ChunkTable make_chunk_table() {
   ChunkTable t{};
   int n = 0, off = 0;
@@ -132,8 +128,8 @@ __host__ __device__ constexpr ChunkTable make_chunk_table() {
         const int src = seg == 0 ? SRC_ENC : (seg == 1 ? SRC_HID : SRC_DIR);
         const int klen = seg == 0 ? (has_enc ? kXyzPad : 0) : (seg == 1 ? (has_hid ? kWidth : 0) : (l == 9 ? kDirPad : 0));
         const int wbase = seg == 0 ? 0 : (seg == 1 ? (has_enc ? kXyzPad : 0) : kWidth);   // padded weight K offset
-        for (int k0 = 0; k0 < klen; k0 += KC) {
-          const int kc = klen - k0 < KC ? klen - k0 : KC;
+        for (int k0 = 0; k0 < klen; k0 += kKc) {
+          const int kc = klen - k0 < kKc ? klen - k0 : kKc;
           Chunk c{};
           c.layer = l; c.half = half; c.src = src; c.a16 = k0 / 16; c.w16 = (wbase + k0) / 16; c.steps = kc / 16;
           c.first = first; c.mid = c.steps; c.off = off;
@@ -171,15 +167,10 @@ __host__ __device__ constexpr ChunkTable make_chunk_table() {
   t.steps_total = off;
   return t;
 }
-__constant__ ChunkTable c_chunks_cg2 = make_chunk_table<128>();
-static constexpr ChunkTable h_chunks_cg2 = make_chunk_table<128>();
-static_assert(h_chunks_cg2.n_total == 35 && h_chunks_cg2.n_sigma_only == 32, "chunk schedule (K128)");
-static_assert(h_chunks_cg2.steps_total == 258, "K16 steps per tile");
-template <int kCg>
-__device__ __forceinline__ const ChunkTable& chunk_table() {
-  static_assert(kCg == 2, "only CTA pairs are built");
-  return c_chunks_cg2;
-}
+__constant__ ChunkTable c_chunks = make_chunk_table();
+static constexpr ChunkTable h_chunks = make_chunk_table();
+static_assert(h_chunks.n_total == 35 && h_chunks.n_sigma_only == 32, "chunk schedule (K128)");
+static_assert(h_chunks.steps_total == 258, "K16 steps per tile");
 
 // number of waits on barrier code `code` (WAIT_*) in chunks [0, ci) -- plus chunk ci's own `wait` when
 // the question is about its mid-chunk wait.  a_ready[q] completes once per layer epilogue, 8 per
@@ -199,7 +190,7 @@ __host__ __device__ constexpr bool wait_counts_ok(const ChunkTable& t) {
   }
   return prior_waits(t, t.n_total, WAIT_ENC, 0) == 1 && prior_waits(t, t.n_total, WAIT_DIR, 0) == 1;
 }
-static_assert(wait_counts_ok(h_chunks_cg2), "static wait parities");
+static_assert(wait_counts_ok(h_chunks), "static wait parities");
 
 template <class F, int... I>
 __device__ __forceinline__ void static_for_impl(F&& f, std::integer_sequence<int, I...>) {
@@ -236,7 +227,7 @@ __host__ __device__ constexpr uint32_t step_image_bytes(int precision) {
 // scratch at the end of the image: W' = Wd[:, :256] Wf (128 x 256) and b' = bd + Wd[:, :256] bf (128)
 constexpr size_t kFusedFloats = (size_t)kHalf * kWidth + kHalf;
 __host__ __device__ constexpr size_t chunks_bytes(int precision) {
-  return (size_t)make_chunk_table<128>().steps_total * step_image_bytes(precision);
+  return (size_t)make_chunk_table().steps_total * step_image_bytes(precision);
 }
 size_t tc_packed_bytes(int precision) {
   return sizeof(PackedHeader) + kConstBytes + chunks_bytes(precision) + kFusedFloats * sizeof(float);
@@ -342,10 +333,8 @@ __device__ __forceinline__ void sincos_fast(float x, float* sn, float* cs) {
 }
 
 // ------------------------------------------------------------------ pack kernel
-using ParamPtrsTc = ParamPtrs;
-
 // W'[n][k] = sum_j Wd[n][j] Wf[j][k],  b'[n] = bd[n] + sum_j Wd[n][j] bf[j]   (double accumulation)
-__global__ void fuse_bottleneck_kernel(ParamPtrsTc pp, float* fused, const PackedHeader* hdr, int only_if_dirty) {
+__global__ void fuse_bottleneck_kernel(ParamPtrs pp, float* fused, const PackedHeader* hdr, int only_if_dirty) {
   if (only_if_dirty && !hdr->dirty) return;
   const float* Wd = pp.p[18];   // (128, 283)
   const float* Wf = pp.p[16];   // (256, 256)
@@ -360,11 +349,10 @@ __global__ void fuse_bottleneck_kernel(ParamPtrsTc pp, float* fused, const Packe
   }
 }
 
-template <bool kBf16, bool kSplit, int kCg>
-__global__ void pack_tc_kernel(ParamPtrsTc pp, int precision, int new_activation, unsigned char* image, int only_if_dirty) {
-  using G = Geo<kCg>;
+template <bool kBf16, bool kSplit>
+__global__ void pack_tc_kernel(ParamPtrs pp, int precision, int new_activation, unsigned char* image, int only_if_dirty) {
   constexpr ConstLayout CL = make_const_layout();
-  const ChunkTable& tab = chunk_table<kCg>();
+  const ChunkTable& tab = c_chunks;
   PackedHeader* hdr = reinterpret_cast<PackedHeader*>(image);
   if (only_if_dirty && !hdr->dirty) return;
   float* cst = reinterpret_cast<float*>(image + sizeof(PackedHeader));
@@ -375,7 +363,6 @@ __global__ void pack_tc_kernel(ParamPtrsTc pp, int precision, int new_activation
     hdr->magic = kMagic;
     hdr->precision = precision;
     hdr->new_activation = new_activation;
-    hdr->cta_group = kCg;
   }
   for (int e = gtid; e < kConstFloats; e += gsz) {
     float v = 0.f;
@@ -407,10 +394,10 @@ __global__ void pack_tc_kernel(ParamPtrsTc pp, int precision, int new_activation
     const int src_k = l == 0 ? 63 : (l == 4 ? 319 : (l == 9 ? 283 : 256));
     float w = col >= 0 ? pp.p[param_weight_index(l)][n * src_k + col] : 0.f;
     if (l == 9 && kpad < kWidth) w = fused[n * kWidth + kpad];     // direction layer sees h8 through W'
-    const int owner = r / G::kRowsB, rr = r - owner * G::kRowsB;
-    const uint32_t part = G::kStepBytes * c.steps;                // bytes of one of {hi, lo} of a share
-    unsigned char* base = chunks + (size_t)c.off * (G::kStepBytes * kParts * kCg) + (size_t)owner * part * kParts;
-    const uint32_t off = (uint32_t)(kk >> 3) * (G::kRowsB * 16) + rr * 16 + (kk & 7) * 2;
+    const int owner = r / kRowsB, rr = r - owner * kRowsB;
+    const uint32_t part = kStepBytes * c.steps;                   // bytes of one of {hi, lo} of a share
+    unsigned char* base = chunks + (size_t)c.off * (kStepBytes * kParts * 2) + (size_t)owner * part * kParts;
+    const uint32_t off = (uint32_t)(kk >> 3) * (kRowsB * 16) + rr * 16 + (kk & 7) * 2;
     if (kSplit) {
       uint16_t hi, lo;
       split16<kBf16>(w, hi, lo);
@@ -422,36 +409,30 @@ __global__ void pack_tc_kernel(ParamPtrsTc pp, int precision, int new_activation
   }
 }
 
-template <int kCg>
-static int launch_pack_tc_cg(const ParamPtrsTc& pp, int precision, int new_activation, unsigned char* img,
-                             int only_if_dirty, cudaStream_t st) {
-  if (precision < SNB_PREC_F16X3 || precision > SNB_PREC_BF16)
-    return fail(SNB_ERR_INVALID, "launch_pack_tc: precision %d is not a tensor-core mode", precision);
+int launch_pack_tc(const float* const* params, int precision, int new_activation, void* image, int only_if_dirty,
+                   cudaStream_t st) {
+  auto pack = precision == SNB_PREC_F16X3    ? pack_tc_kernel<false, true>
+              : precision == SNB_PREC_BF16X3 ? pack_tc_kernel<true, true>
+              : precision == SNB_PREC_BF16   ? pack_tc_kernel<true, false>
+                                             : nullptr;
+  if (!pack) return fail(SNB_ERR_INVALID, "launch_pack_tc: precision %d is not a tensor-core mode", precision);
+  ParamPtrs pp;
+  for (int i = 0; i < SNB_N_PARAM_TENSORS; ++i) pp.p[i] = params[i];
+  unsigned char* img = reinterpret_cast<unsigned char*>(image);
   float* fused = reinterpret_cast<float*>(img + sizeof(PackedHeader) + kConstBytes + chunks_bytes(precision));
   fuse_bottleneck_kernel<<<148, 256, 0, st>>>(pp, fused, reinterpret_cast<const PackedHeader*>(img), only_if_dirty);
   if (int rc = check_launch("fuse_bottleneck_kernel")) return rc;
-  if (precision == SNB_PREC_F16X3) pack_tc_kernel<false, true, kCg><<<296, 256, 0, st>>>(pp, precision, new_activation, img, only_if_dirty);
-  else if (precision == SNB_PREC_BF16X3) pack_tc_kernel<true, true, kCg><<<296, 256, 0, st>>>(pp, precision, new_activation, img, only_if_dirty);
-  else if (precision == SNB_PREC_BF16) pack_tc_kernel<true, false, kCg><<<296, 256, 0, st>>>(pp, precision, new_activation, img, only_if_dirty);
-  else return fail(SNB_ERR_INVALID, "launch_pack_tc: precision %d is not a tensor-core mode", precision);
+  pack<<<296, 256, 0, st>>>(pp, precision, new_activation, img, only_if_dirty);
   return check_launch("pack_tc_kernel");
-}
-
-int launch_pack_tc(const float* const* params, int precision, int new_activation, void* image, int only_if_dirty,
-                   cudaStream_t st) {
-  ParamPtrsTc pp;
-  for (int i = 0; i < SNB_N_PARAM_TENSORS; ++i) pp.p[i] = params[i];
-  unsigned char* img = reinterpret_cast<unsigned char*>(image);
-  return launch_pack_tc_cg<2>(pp, precision, new_activation, img, only_if_dirty, st);
 }
 
 // ------------------------------------------------------------------ shared memory
 // kTrain: 0 = inference, 1 = training forward keeping fp32 row-major activations (snb_field_forward_train),
 //         2 = training forward keeping fp16 activations in the T32 layout + ReLU mask words (act16.cuh)
-template <bool kSplit, int kCg, int kTrain = 0>
+template <bool kSplit, int kTrain>
 struct TcSmem {
   static constexpr int kParts = kSplit ? 2 : 1;
-  static constexpr uint32_t kStageBytes = Geo<kCg>::kPartBytesMax * kParts;   // this CTA's share of a full chunk
+  static constexpr uint32_t kStageBytes = kPartBytesMax * kParts;   // this CTA's share of a full chunk
   // up to 160 KB of weights in flight; the training forward gives 64 KB of that to the store tiles below
   static constexpr int kStagesRaw = ((kTrain == 1 ? 96 : 160) * 1024) / kStageBytes;
   static constexpr int kStages = kStagesRaw > 16 ? 16 : kStagesRaw;
@@ -510,14 +491,10 @@ __device__ __forceinline__ void trace(bool on, int idx) { if (on && idx < kTrace
 
 __device__ __forceinline__ void epi_bar_sync() { asm volatile("bar.sync 1, 512;" ::: "memory"); }
 
-// canonical (SWIZZLE_NONE, K-major) byte offset of element (row, k) in a [k8][128 rows][8] block
-__device__ __forceinline__ uint32_t canon_off(int row, int k) { return (uint32_t)(k >> 3) * (kTile * 16) + row * 16 + (k & 7) * 2; }
-
-template <bool kBf16, bool kSplit, bool kEmbedded, int kCg, int kTrain = 0>
+template <bool kBf16, bool kSplit, bool kEmbedded, int kTrain>
 __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
   static_assert(!(kTrain != 0 && kEmbedded), "the training forward is the fused (rays, z) entry only");
-  using Smem = TcSmem<kSplit, kCg, kTrain>;
-  using G = Geo<kCg>;
+  using Smem = TcSmem<kSplit, kTrain>;
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   Smem& s = *reinterpret_cast<Smem*>(smem_raw);
   constexpr ConstLayout CL = make_const_layout();
@@ -525,19 +502,19 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
   constexpr int kStages = Smem::kStages;
   constexpr int kParts = Smem::kParts;
   static_assert(kStages <= 16, "barrier arrays");
-  const ChunkTable& tab = chunk_table<kCg>();
+  const ChunkTable& tab = c_chunks;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const PackedHeader* hdr = reinterpret_cast<const PackedHeader*>(p.image);
   const int new_activation = hdr->new_activation;
   const float* g_cst = reinterpret_cast<const float*>(p.image + sizeof(PackedHeader));
   const unsigned char* g_chunks = p.image + sizeof(PackedHeader) + kConstBytes;
-  const uint32_t cta_rank = kCg == 2 ? cluster_ctarank() : 0;
+  const uint32_t cta_rank = cluster_ctarank();
   const bool leader = cta_rank == 0;
-  // tile slots: group g (a CTA or a CTA pair) handles tile (g + i * n_groups) * kCg + rank.  Every
-  // CTA of a group runs the same number of slots; slots past the end compute on zeros, store nothing.
+  // tile slots: pair g handles tile (g + i * n_pairs) * 2 + rank.  Both CTAs of a pair run the same
+  // number of slots; slots past the end compute on zeros, store nothing.
   const long long ntiles = (p.n_points + kTile - 1) / kTile;
-  const long long n_groups = gridDim.x / kCg, group = blockIdx.x / kCg;
-  const long long n_slots = ((ntiles + kCg - 1) / kCg + n_groups - 1) / n_groups;
+  const long long n_pairs = gridDim.x / 2, pair = blockIdx.x / 2;
+  const long long n_slots = ((ntiles + 1) / 2 + n_pairs - 1) / n_pairs;
   const int n_layers_epi = 8;   // trunk layers with a TMEM->TMEM epilogue (the bottleneck is folded away)
   const int n_chunks = p.sigma_only ? tab.n_sigma_only : tab.n_total;
   // Deferred direction-layer epilogue (round 2, single-product mode).  The 128 softplus + rgb head of a tile are
@@ -557,31 +534,31 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
   // ---------------- one-time setup
   for (int i = tid; i < kConstFloats; i += kThreads) s.cst[i] = g_cst[i];
   if (tid == 0) {
-    // full: this CTA's loader (+ the peer's relay, at the leader of a pair); a_ready / enc_ready live
-    // at the leader and count the epilogue threads of every CTA of the group
-    for (int i = 0; i < kStages; ++i) { mbar_init(&s.full[i], (kCg == 2 && leader) ? 2 : 1); mbar_init(&s.empty[i], 1); }
+    // full: this CTA's loader (+ the peer's relay, at the leader); a_ready / enc_ready live at the
+    // leader and count the epilogue threads of both CTAs
+    for (int i = 0; i < kStages; ++i) { mbar_init(&s.full[i], leader ? 2 : 1); mbar_init(&s.empty[i], 1); }
     mbar_init(&s.d_full[0], 1); mbar_init(&s.d_full[1], 1); mbar_init(&s.a_free, 1);
-    for (int i = 0; i < 4; ++i) mbar_init(&s.a_ready[i], kEpiWarps * 16 * kCg);   // the two warps-of-four that own the quarter
-    mbar_init(&s.enc_ready, kEncWarps * 32 * kCg);
-    mbar_init(&s.dir_ready, kEncWarps * 32 * kCg);
-    mbar_init(&s.d_drained, kEpiWarps * 32 * kCg);
+    for (int i = 0; i < 4; ++i) mbar_init(&s.a_ready[i], kEpiWarps * 16 * 2);   // the two warps-of-four that own the quarter
+    mbar_init(&s.enc_ready, kEncWarps * 32 * 2);
+    mbar_init(&s.dir_ready, kEncWarps * 32 * 2);
+    mbar_init(&s.d_drained, kEpiWarps * 32 * 2);
     mbar_init(&s.enc_free, 1);
     mbar_init(&s.dir_free, 1);
     mbar_init(&s.rgb_done, kEpiWarps);
     mbar_init(&s.d_full_dir, 1);
     fence_mbar_init();
   }
-  if (warp == kMmaWarp) { if (kCg == 2) tmem_alloc_pair(&s.tmem_base); else tmem_alloc<512>(&s.tmem_base); }
+  if (warp == kMmaWarp) tmem_alloc_pair(&s.tmem_base);
   tc_fence_before();
   __syncthreads();
-  if (kCg == 2) cluster_sync_all();   // the peer's barriers exist before anyone signals them
+  cluster_sync_all();   // the peer's barriers exist before anyone signals them
   tc_fence_after();
   const uint32_t tbase = s.tmem_base;
 
   // ---- helpers shared by the encoder and the epilogue warps
-  auto tile_of = [&](long long slot) { return (group + slot * n_groups) * kCg + cta_rank; };
+  auto tile_of = [&](long long slot) { return (pair + slot * n_pairs) * 2 + cta_rank; };
   // hand-off to the MMA issuer, which lives in the leader CTA
-  auto signal = [&](uint64_t* bar) { if (kCg == 2 && !leader) mbar_arrive_remote(bar, 0); else mbar_arrive(bar); };
+  auto signal = [&](uint64_t* bar) { if (!leader) mbar_arrive_remote(bar, 0); else mbar_arrive(bar); };
   // 16-bit storage: 8 consecutive features of one point -> one 16-byte cell of a T32 tensor
   auto store_cell16 = [&](unsigned char* base, long long pt, int f8, int F, const float (&v)[8]) {
     if (pt >= p.ppad) return;
@@ -600,30 +577,6 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
     *reinterpret_cast<uint4*>(hi_base + off) = make_uint4(h[0], h[1], h[2], h[3]);
     if (kSplit) *reinterpret_cast<uint4*>(lo_base + off) = make_uint4(l[0], l[1], l[2], l[3]);
   };
-  // 8 consecutive channels [c_lo, c_lo+8) of Embedding(3, L)(x): [x(3), sin(2^0 x)(3), cos(2^0 x)(3),
-  // sin(2^1 x)(3), ...] (nerf.py:36-41), one sincos per (frequency, coordinate) that the window touches
-  auto embed8 = [&](const float (&x)[3], int c_lo, int n_ch, int n_freqs, float (&v)[8]) {
-#pragma unroll
-    for (int j = 0; j < 8; ++j) v[j] = (c_lo + j < 3) ? x[(c_lo + j) % 3] : 0.f;   // identity / zero pad
-    for (int f = 0; f < n_freqs; ++f) {
-      const int base = 3 + 6 * f;
-      if (base + 6 <= c_lo || base >= c_lo + 8) continue;
-#pragma unroll
-      for (int c = 0; c < 3; ++c) {
-        const int js = base + c - c_lo, jc = js + 3;
-        if ((js >= 0 && js < 8) || (jc >= 0 && jc < 8)) {
-          float sn, cs;
-          if (kSplit) sincosf(x[c] * (float)(1 << f), &sn, &cs);
-          else sincos_fast(x[c] * (float)(1 << f), &sn, &cs);
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {           // static indices keep v[] in registers
-            if (j == js) v[j] = sn;
-            if (j == jc && base + 3 + c < n_ch) v[j] = cs;
-          }
-        }
-      }
-    }
-  };
 
   if (warp == kLoadWarp) {
     // ======================= weight loader (one elected lane) =======================
@@ -635,8 +588,8 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
           const uint32_t st = it % kStages, ph = (it / kStages) & 1;
           mbar_wait(&s.empty[st], ph ^ 1);
           const Chunk c = tab.c[ci];
-          const uint32_t share = G::kStepBytes * kParts * c.steps;      // this CTA's bytes of the chunk
-          const unsigned char* src = g_chunks + (size_t)c.off * (G::kStepBytes * kParts * kCg) + (size_t)cta_rank * share;
+          const uint32_t share = kStepBytes * kParts * c.steps;         // this CTA's bytes of the chunk
+          const unsigned char* src = g_chunks + (size_t)c.off * (kStepBytes * kParts * 2) + (size_t)cta_rank * share;
           mbar_arrive_expect_tx(&s.full[st], share);
           for (uint32_t o = 0; o < share; o += 16384)
             bulk_g2s(s.ring[st] + o, src + o, share - o < 16384 ? share - o : 16384, &s.full[st]);
@@ -665,20 +618,19 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
     // more than the 515 cycles the tensor pipe needs for a bf16 chunk -- the issuer, not the
     // pipe, set the pace; profiles/r01_timing_experiments.txt v11.)
     if (elect_one()) {
-      constexpr ChunkTable T = make_chunk_table<G::kKc>();
-      const uint32_t idesc = make_idesc(kBf16 ? kFmtBF16 : kFmtF16, kTile * kCg, kNh);
+      constexpr ChunkTable T = make_chunk_table();
+      const uint32_t idesc = make_idesc(kBf16 ? kFmtBF16 : kFmtF16, 2 * kTile, kNh);   // M = both tiles of the pair
       const uint32_t enc_hi = smem_u32(s.enc[0]), dir_hi = smem_u32(s.dir[0]);
       const uint32_t enc_lo = smem_u32(s.enc[kSplit ? 1 : 0]), dir_lo = smem_u32(s.dir[kSplit ? 1 : 0]);
       // descriptors as (lo, hi) words: only the 14-bit start-address field in the low word moves
-      const uint64_t desc_b0 = make_smem_desc(0, G::kRowsB * 16, 128);
+      const uint64_t desc_b0 = make_smem_desc(0, kRowsB * 16, 128);
       const uint64_t desc_a0 = make_smem_desc(0, kTile * 16, 128);
       const uint32_t bd_hi32 = (uint32_t)(desc_b0 >> 32), ad_hi32 = (uint32_t)(desc_a0 >> 32);
       const uint32_t b_ring0 = (uint32_t)desc_b0 + (smem_u32(s.ring[0]) >> 4);
       const uint32_t a_enc_hi = (uint32_t)desc_a0 + (enc_hi >> 4), a_enc_lo = (uint32_t)desc_a0 + (enc_lo >> 4);
       const uint32_t a_dir_hi = (uint32_t)desc_a0 + (dir_hi >> 4), a_dir_lo = (uint32_t)desc_a0 + (dir_lo >> 4);
-      constexpr uint32_t kStepB = (2 * G::kRowsB * 16) >> 4;     // one K16 step inside a chunk, in 16-B units
+      constexpr uint32_t kStepB = (2 * kRowsB * 16) >> 4;        // one K16 step inside a chunk, in 16-B units
       constexpr uint32_t kStepA = (2 * kTile * 16) >> 4;
-      auto commit = [&](uint64_t* bar) { if (kCg == 2) mma2_commit(bar); else mma_commit(bar); };
       uint32_t st = 0, ph_full = 0;            // ring position: stage and the parity of its `full` barrier
       for (long long slot = 0; slot < n_slots; ++slot) {
         const uint32_t slot_par = (uint32_t)slot & 1;    // enc_ready / dir_ready / d_drained complete once per slot
@@ -703,7 +655,7 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
           trace(tr, CI * 4 + 2);
           const uint32_t d = tbase + (c.layer == 9 ? (kDirTmem ? kColAlo : kColD) : kColD + c.half * kNh);
           const uint32_t bh = b_ring0 + st * (kStageBytes >> 4);           // W_hi block
-          const uint32_t bl = bh + ((G::kStepBytes * c.steps) >> 4);        // W_lo block
+          const uint32_t bl = bh + ((kStepBytes * c.steps) >> 4);           // W_lo block
           // K16 steps [kLo, kHi) of this chunk
           auto issue_range = [&](auto lo_tag, auto hi_tag) {
             constexpr int kLo = decltype(lo_tag)::value, kHi = decltype(hi_tag)::value;
@@ -713,16 +665,10 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
 #pragma unroll
               for (int ks = kLo; ks < kHi; ++ks) {
                 const uint32_t acc = (ks == 0 && c.first) ? 0u : 1u;
-                if (kCg == 2) {
-                  mma2_ts_lohi(d, a_hi + ks * 8, bh + ks * kStepB, bd_hi32, idesc, acc);
-                  if (kSplit) {
-                    mma2_ts_lohi(d, a_lo + ks * 8, bh + ks * kStepB, bd_hi32, idesc, 1);
-                    mma2_ts_lohi(d, a_hi + ks * 8, bl + ks * kStepB, bd_hi32, idesc, 1);
-                  }
-                } else {
-                  const uint64_t b1 = ((uint64_t)bd_hi32 << 32) | (bh + ks * kStepB), b2 = ((uint64_t)bd_hi32 << 32) | (bl + ks * kStepB);
-                  mma_ts(d, a_hi + ks * 8, b1, idesc, acc);
-                  if (kSplit) { mma_ts(d, a_lo + ks * 8, b1, idesc, 1); mma_ts(d, a_hi + ks * 8, b2, idesc, 1); }
+                mma2_ts_lohi(d, a_hi + ks * 8, bh + ks * kStepB, bd_hi32, idesc, acc);
+                if (kSplit) {
+                  mma2_ts_lohi(d, a_lo + ks * 8, bh + ks * kStepB, bd_hi32, idesc, 1);
+                  mma2_ts_lohi(d, a_hi + ks * 8, bl + ks * kStepB, bd_hi32, idesc, 1);
                 }
               }
             } else {
@@ -732,17 +678,10 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
 #pragma unroll
               for (int ks = kLo; ks < kHi; ++ks) {
                 const uint32_t acc = (ks == 0 && c.first) ? 0u : 1u;
-                if (kCg == 2) {
-                  mma2_ss_lohi(d, ah + ks * kStepA, ad_hi32, bh + ks * kStepB, bd_hi32, idesc, acc);
-                  if (kSplit) {
-                    mma2_ss_lohi(d, al + ks * kStepA, ad_hi32, bh + ks * kStepB, bd_hi32, idesc, 1);
-                    mma2_ss_lohi(d, ah + ks * kStepA, ad_hi32, bl + ks * kStepB, bd_hi32, idesc, 1);
-                  }
-                } else {
-                  const uint64_t a1 = ((uint64_t)ad_hi32 << 32) | (ah + ks * kStepA), a2 = ((uint64_t)ad_hi32 << 32) | (al + ks * kStepA);
-                  const uint64_t b1 = ((uint64_t)bd_hi32 << 32) | (bh + ks * kStepB), b2 = ((uint64_t)bd_hi32 << 32) | (bl + ks * kStepB);
-                  mma_ss(d, a1, b1, idesc, acc);
-                  if (kSplit) { mma_ss(d, a2, b1, idesc, 1); mma_ss(d, a1, b2, idesc, 1); }
+                mma2_ss_lohi(d, ah + ks * kStepA, ad_hi32, bh + ks * kStepB, bd_hi32, idesc, acc);
+                if (kSplit) {
+                  mma2_ss_lohi(d, al + ks * kStepA, ad_hi32, bh + ks * kStepB, bd_hi32, idesc, 1);
+                  mma2_ss_lohi(d, ah + ks * kStepA, ad_hi32, bl + ks * kStepB, bd_hi32, idesc, 1);
                 }
               }
             }
@@ -758,13 +697,13 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
             issue_range(IM{}, IS{});
             trace(tr, 512 + CI * 4 + 1);
           }
-          commit(&s.empty[st]);        // ring slot free (in both CTAs of a pair) once these MMAs retire
+          mma2_commit(&s.empty[st]);   // ring slot free (in both CTAs of the pair) once these MMAs retire
           trace(tr, 512 + CI * 4 + 2);
-          if (c.commit & COMMIT_AFREE) commit(&s.a_free);
-          if (c.commit & COMMIT_D0) commit((c.layer == 9 && kDirTmem) ? &s.d_full_dir : &s.d_full[0]);
-          if (c.commit & COMMIT_D1) commit(&s.d_full[1]);
-          if (c.src == SRC_ENC && c.layer == 4 && c.half == 1) commit(&s.enc_free);   // last reader of enc in this slot
-          if (c.src == SRC_DIR) commit(&s.dir_free);
+          if (c.commit & COMMIT_AFREE) mma2_commit(&s.a_free);
+          if (c.commit & COMMIT_D0) mma2_commit((c.layer == 9 && kDirTmem) ? &s.d_full_dir : &s.d_full[0]);
+          if (c.commit & COMMIT_D1) mma2_commit(&s.d_full[1]);
+          if (c.src == SRC_ENC && c.layer == 4 && c.half == 1) mma2_commit(&s.enc_free);   // last reader of enc in this slot
+          if (c.src == SRC_DIR) mma2_commit(&s.dir_free);
           trace(tr, 512 + CI * 4 + 3);
           if (++st == kStages) { st = 0; ph_full ^= 1; }
           trace(tr, CI * 4 + 3);
@@ -985,7 +924,6 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
       const long long pt = pt_slot;
       for (int l = 0; l < n_layers_epi; ++l) {
         const float* bias = s.cst + CL.b[l];
-        const bool relu = true;
 #pragma unroll 1
         for (int h = 0; h < 2; ++h) {
           const bool tr = (p.debug & 8) && blockIdx.x == 0 && slot == 3 && tid == 0;
@@ -1002,8 +940,8 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
           trace(tr, tb + 2);
           // bias + activation + hi/lo split, in place: v[2j] = hi pair j, v[2j+1] = lo pair j
           uint32_t mask_word = 0;        // kTrain == 2: [value > 0] of this thread's 32 columns, stored after the hand-off
-          auto finish_group = [&](auto relu_tag, auto sigma_tag) {
-            constexpr bool kRelu = decltype(relu_tag)::value, kSigma = decltype(sigma_tag)::value;
+          auto finish_group = [&](auto sigma_tag) {
+            constexpr bool kSigma = decltype(sigma_tag)::value;
             const float2* b2 = reinterpret_cast<const float2*>(bias + c0);
             const float2* w2 = reinterpret_cast<const float2*>(s.cst + CL.sigma_w + c0);
             const long long pt_block0 = pt - lane;      // first row of this warp's 32-row block
@@ -1014,7 +952,7 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
 #pragma unroll
             for (int j = 0; j < 16; j += 2) {
               float x[4];
-              if (kRelu && !kSigma && kTrain == 0) {
+              if (!kSigma && kTrain == 0) {
                 // nobody needs the fp32 post-activation value: ReLU and the fp16 range guard ride on the converts
                 // one 16-byte bias load and two packed fp32x2 adds (FADD2) per four columns
                 const float4 bb = *reinterpret_cast<const float4*>(b2 + j);
@@ -1031,17 +969,15 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
                 const float2 x01 = __fadd2_rn(make_float2(__uint_as_float(v[2 * j]), __uint_as_float(v[2 * j + 1])), make_float2(bb.x, bb.y));
                 const float2 x23 = __fadd2_rn(make_float2(__uint_as_float(v[2 * j + 2]), __uint_as_float(v[2 * j + 3])), make_float2(bb.z, bb.w));
                 x[0] = x01.x; x[1] = x01.y; x[2] = x23.x; x[3] = x23.y;
-                if (kRelu) {
 #pragma unroll
-                  for (int e = 0; e < 4; ++e) x[e] = fmaxf(x[e], 0.f);
-                }
+                for (int e = 0; e < 4; ++e) x[e] = fmaxf(x[e], 0.f);
               } else {
 #pragma unroll
                 for (int e = 0; e < 2; ++e) {
                   const float2 bb = b2[j + e];
                   x[2 * e] = __uint_as_float(v[2 * (j + e)]) + bb.x;
                   x[2 * e + 1] = __uint_as_float(v[2 * (j + e) + 1]) + bb.y;
-                  if (kRelu) { x[2 * e] = fmaxf(x[2 * e], 0.f); x[2 * e + 1] = fmaxf(x[2 * e + 1], 0.f); }
+                  x[2 * e] = fmaxf(x[2 * e], 0.f); x[2 * e + 1] = fmaxf(x[2 * e + 1], 0.f);
                   if (kSigma) {
                     const float2 ww = w2[j + e];
                     sig_part = fmaf(x[2 * e], ww.x, sig_part); sig_part = fmaf(x[2 * e + 1], ww.y, sig_part);
@@ -1052,8 +988,8 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
                 keep[(j >> 1) & 3] = make_float4(x[0], x[1], x[2], x[3]);
                 if (((j >> 1) & 3) == 3) store_block16(keep, save_blk + (j >> 3) * 16, kWidth, pt_block0);
               }
-              split_pair<kBf16, kSplit, kRelu>(x[0], x[1], v[2 * j], v[2 * j + 1]);
-              split_pair<kBf16, kSplit, kRelu>(x[2], x[3], v[2 * j + 2], v[2 * j + 3]);
+              split_pair<kBf16, kSplit, true>(x[0], x[1], v[2 * j], v[2 * j + 1]);
+              split_pair<kBf16, kSplit, true>(x[2], x[3], v[2 * j + 2], v[2 * j + 3]);
               if (kTrain == 2) {
                 // fp16 modes: the hi word of the split IS rn_fp16(value) (saturated); bf16 modes convert separately
                 h16[j] = kBf16 ? pack_half2_sat(x[0], x[1]) : v[2 * j];
@@ -1076,8 +1012,8 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
             }
             mask_word = mword;
           };
-          if (l == 7) finish_group(std::true_type{}, std::true_type{});
-          else finish_group(std::true_type{}, std::false_type{});
+          if (l == 7) finish_group(std::true_type{});
+          else finish_group(std::false_type{});
           // half a's results go to A[k 0..127], which this layer's (b,k0) MMAs still read: the math above
           // overlaps both b phases, the stores wait until those MMAs have retired (a_free); half b's
           // target A[k 128..255] is idle
@@ -1171,33 +1107,33 @@ __global__ void __launch_bounds__(kThreads, 1) field_tc_kernel(TcParams p) {
   }
   tc_fence_before();
   __syncthreads();
-  if (kCg == 2) cluster_sync_all();   // neither CTA leaves (or frees TMEM) while its peer may still touch it
-  if (warp == kMmaWarp) { if (kCg == 2) tmem_dealloc_pair(tbase); else tmem_dealloc<512>(tbase); }
+  cluster_sync_all();   // neither CTA leaves (or frees TMEM) while its peer may still touch it
+  if (warp == kMmaWarp) tmem_dealloc_pair(tbase);
 }
 
 // ------------------------------------------------------------------ host
-template <bool kBf16, bool kSplit, bool kEmbedded, int kCg, int kTrain = 0>
+template <bool kBf16, bool kSplit, bool kEmbedded, int kTrain>
 static int launch_tc(const TcParams& p, cudaStream_t st) {
   static SmemOptIn optin;
   const long long ntiles = (p.n_points + kTile - 1) / kTile;
   if (ntiles == 0) return SNB_OK;       // an empty pass is a no-op: no CUDA call at all
-  const size_t smem = sizeof(TcSmem<kSplit, kCg, kTrain>) + 1024;
-  auto kern = field_tc_kernel<kBf16, kSplit, kEmbedded, kCg, kTrain>;
+  const size_t smem = sizeof(TcSmem<kSplit, kTrain>) + 1024;
+  auto kern = field_tc_kernel<kBf16, kSplit, kEmbedded, kTrain>;
   if (int rc = ensure_smem(kern, optin, (int)smem, "field_tc")) return rc;
   const int sms = sm_count();
-  long long groups = (ntiles + kCg - 1) / kCg;
-  if (groups > sms / kCg) groups = sms / kCg;
+  long long pairs = (ntiles + 1) / 2;
+  if (pairs > sms / 2) pairs = sms / 2;
   static const int debug = getenv("SNB_TC_DEBUG") ? atoi(getenv("SNB_TC_DEBUG")) : 0;
   TcParams pd = p;
   pd.debug = debug;
   cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)(groups * kCg));
+  cfg.gridDim = dim3((unsigned)(pairs * 2));
   cfg.blockDim = dim3(kThreads);
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = kCg;
+  attr[0].val.clusterDim.x = 2;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
@@ -1207,17 +1143,12 @@ static int launch_tc(const TcParams& p, cudaStream_t st) {
   return check_launch("field_tc_kernel");
 }
 
-template <bool kBf16, bool kSplit, bool kEmbedded>
-static int launch_tc_cg(const TcParams& p, cudaStream_t st) {
-  return launch_tc<kBf16, kSplit, kEmbedded, 2>(p, st);
-}
-
-template <bool kEmbedded>
+template <bool kEmbedded, int kTrain>
 static int dispatch_tc(int precision, const TcParams& p, cudaStream_t st) {
   switch (precision) {
-    case SNB_PREC_F16X3: return launch_tc_cg<false, true, kEmbedded>(p, st);
-    case SNB_PREC_BF16X3: return launch_tc_cg<true, true, kEmbedded>(p, st);
-    case SNB_PREC_BF16: return launch_tc_cg<true, false, kEmbedded>(p, st);
+    case SNB_PREC_F16X3: return launch_tc<false, true, kEmbedded, kTrain>(p, st);
+    case SNB_PREC_BF16X3: return launch_tc<true, true, kEmbedded, kTrain>(p, st);
+    case SNB_PREC_BF16: return launch_tc<true, false, kEmbedded, kTrain>(p, st);
   }
   return fail(SNB_ERR_INVALID, "precision %d is not a tensor-core mode", precision);
 }
@@ -1230,7 +1161,7 @@ int field_forward_tc(const void* packed, int precision, const float* rays, const
   p.n_points = (long long)n_rays * n_samples;
   p.sigma_only = sigma_only;
   p.out = raw;
-  return dispatch_tc<false>(precision, p, st);
+  return dispatch_tc<false, 0>(precision, p, st);
 }
 
 int field_forward_train_tc(const void* packed, int precision, const float* rays, const float* z, int64_t n_rays,
@@ -1242,12 +1173,7 @@ int field_forward_train_tc(const void* packed, int precision, const float* rays,
   p.n_points = (long long)n_rays * n_samples;
   p.out = raw;
   p.save_enc = save_enc; p.save_dir = save_dir; p.save_h = save_h; p.save_g = save_g;
-  switch (precision) {
-    case SNB_PREC_F16X3: return launch_tc<false, true, false, 2, 1>(p, st);
-    case SNB_PREC_BF16X3: return launch_tc<true, true, false, 2, 1>(p, st);
-    case SNB_PREC_BF16: return launch_tc<true, false, false, 2, 1>(p, st);
-  }
-  return fail(SNB_ERR_INVALID, "precision %d is not a tensor-core mode", precision);
+  return dispatch_tc<false, 1>(precision, p, st);
 }
 
 // training forward with 16-bit activation storage (act16.cuh): `act16` = one buffer of make_act16_layout(P).total bytes
@@ -1263,12 +1189,7 @@ int field_forward_train16_tc(const void* packed, int precision, const float* ray
   p.a_enc = b + L.enc; p.a_dir = b + L.dir; p.a_h = b + L.h[0]; p.a_g = b + L.g;
   p.a_mask = reinterpret_cast<uint32_t*>(b + L.mask);
   p.ppad = a16_pad(p.n_points);
-  switch (precision) {
-    case SNB_PREC_F16X3: return launch_tc<false, true, false, 2, 2>(p, st);
-    case SNB_PREC_BF16X3: return launch_tc<true, true, false, 2, 2>(p, st);
-    case SNB_PREC_BF16: return launch_tc<true, false, false, 2, 2>(p, st);
-  }
-  return fail(SNB_ERR_INVALID, "precision %d is not a tensor-core mode", precision);
+  return dispatch_tc<false, 2>(precision, p, st);
 }
 
 int mlp_forward_tc(const void* packed, int precision, const float* x, int64_t x_stride, int64_t n_points,
@@ -1279,7 +1200,7 @@ int mlp_forward_tc(const void* packed, int precision, const float* x, int64_t x_
   p.n_points = n_points;
   p.sigma_only = sigma_only;
   p.out = out;
-  return dispatch_tc<true>(precision, p, st);
+  return dispatch_tc<true, 0>(precision, p, st);
 }
 
 }  // namespace snb

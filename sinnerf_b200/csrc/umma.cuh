@@ -115,14 +115,6 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
       : "r"(taddr)
       : "memory");
 }
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : SNB_R8(v, 0), SNB_R8(v, 8)
-      : "r"(taddr)
-      : "memory");
-}
 __device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
   asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
                : SNB_R8(v, 0)
@@ -143,11 +135,6 @@ __device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&v)[16
       "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15};" ::SNB_W8(v, 0),
       SNB_W8(v, 8), "r"(taddr)
       : "memory");
-}
-__device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&v)[8]) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%8], {%0, %1, %2, %3, %4, %5, %6, %7};" ::SNB_W8(v, 0),
-               "r"(taddr)
-               : "memory");
 }
 
 // ------------------------------------------------------------------ descriptors
